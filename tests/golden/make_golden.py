@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Generate tests/golden/*.npz in the authoring container (needs /root/reference for the meshes).
+"""Generate tests/golden/p3_scene.npz and synth.npz (the P3 meshes come from tests/golden/reference_models.npz).
 
   p3_scene.npz : the reference's own P3 scene (P3/main.cpp:688-701: Stanford bunny + quad floor + emissive
                  sphere, read with OUR readObj/buildBVHwithSAH restatement), encoded arrays (float16-free,
@@ -12,6 +12,7 @@ The frames that pin it to the reference's own shader source are in refshader.npz
 """
 import os
 import sys
+import tempfile
 import zlib
 
 import numpy as np
@@ -20,8 +21,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 from ezrt_b200 import api, scenes  # noqa: E402
 from tests import oracle_binding as oracle  # noqa: E402
+from tests import reference_golden as rg  # noqa: E402
 
-P3 = "/root/reference/part 3 -- OpenGL Raytracing/source code"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -30,14 +31,15 @@ def crc(a):
 
 
 def p3_scene(builder=api.BVH_SAH_FAST):
-    tl = api.TriangleList()
-    m = api.Material(baseColor=(1, 1, 1))
-    tl.read_obj(P3 + "/models/Stanford Bunny.obj", m, api.transform_matrix((0, 0, 0), (0.3, -1.6, 0), (1.5, 1.5, 1.5)), True)
-    m = api.Material(baseColor=(0.725, 0.71, 0.68))
-    tl.read_obj(P3 + "/models/quad.obj", m, api.transform_matrix((0, 0, 0), (0, -1.4, 0), (18.83, 0.01, 18.83)), False)
-    m = api.Material(baseColor=(1, 1, 1), emissive=(30, 20, 10))
-    tl.read_obj(P3 + "/models/sphere.obj", m, api.transform_matrix((0, 0, 0), (0.0, 0.9, 0.0), (1, 1, 1)), False)
-    return tl.build_bvh(8, builder)
+    with tempfile.TemporaryDirectory() as d:
+        tl = api.TriangleList()
+        m = api.Material(baseColor=(1, 1, 1))
+        tl.read_obj(rg.write_model(d, "p3_bunny"), m, api.transform_matrix((0, 0, 0), (0.3, -1.6, 0), (1.5, 1.5, 1.5)), True)
+        m = api.Material(baseColor=(0.725, 0.71, 0.68))
+        tl.read_obj(rg.write_model(d, "p3_quad"), m, api.transform_matrix((0, 0, 0), (0, -1.4, 0), (18.83, 0.01, 18.83)), False)
+        m = api.Material(baseColor=(1, 1, 1), emissive=(30, 20, 10))
+        tl.read_obj(rg.write_model(d, "p3_sphere"), m, api.transform_matrix((0, 0, 0), (0.0, 0.9, 0.0), (1, 1, 1)), False)
+        return tl.build_bvh(8, builder)
 
 
 def images(tris, nodes, eye, cam, hdr, cache, w=48, h=32, spp=2):

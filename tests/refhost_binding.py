@@ -45,9 +45,9 @@ def transform_matrix(rotate, translate, scale):
     return out
 
 
-def build_scene(meshes, leaf_n=8, sah=True):
-    """meshes: [(obj path, material18, trans16, smooth)] -> (tris [n,36], nodes [m,12]) as main() would upload them"""
-    lib = _load()
+def build_scene(meshes, leaf_n=8, sah=True, part=5):
+    """meshes: [(obj path, material18, trans16, smooth)] -> (tris [n,36], nodes [m,12]) as main() of tutorial `part` would upload them"""
+    lib = _load(part)
     lib.refhost_reset()
     for path, material, trans, smooth in meshes:
         m = np.ascontiguousarray(material, np.float32); t = np.ascontiguousarray(trans, np.float32)

@@ -7,8 +7,9 @@ import zlib
 
 import numpy as np
 
+from tests import reference_golden as rg
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-P5_FSH = "/root/reference/part 5 -- Importance Sampling & Low Discrepancy Sequence/source code/shaders/fshader.fsh"
 
 
 def _table():
@@ -44,11 +45,8 @@ def test_sobol_table_checksum_and_reference_literal():
     t = _table()
     assert len(t) == 256
     assert zlib.crc32(struct.pack("<256I", *t)) == 0xAB08B2B2
-    if os.path.exists(P5_FSH):  # only in the authoring container
-        src = open(P5_FSH).read()
-        m = re.search(r"const uint V\[8\*32\] = \{\s*([0-9u,\s]+)\};", src)
-        ref = [int(x.strip().rstrip("u")) for x in m.group(1).split(",") if x.strip()]
-        assert ref == t
+    # the literal `const uint V[8*32]` of P5's fshader.fsh, as tests/golden/make_golden_reference.py read it
+    assert [int(v) for v in rg.load()["sobol_V"]] == t
 
 
 def test_cranley_patterson_seed_and_wrap(oracle):
